@@ -17,6 +17,11 @@ without the NCCL gather of the observation tensor.  Weak scaling: the same workl
   value  whole-job obs/s with the action masks already resident in HBM and the obs tensor left in HBM
   e2e    the same metric through the public host-buffer call (mv_set_actions + mv_step): H2D actions and D2H
          obs/rewards/dones inside the timed region
+
+--steps K sets every timed loop to K steps.  --dump-outputs DIR writes, after the headline's timed steps, what its last step
+handed the caller (see dump_outputs).  The inputs (env seeds, action stream) depend only on the arguments, so two builds can be
+compared output for output.  The bench loads the native libraries already built in the tree (`python -m megaverse_b200._build`)
+and writes nothing there.
 """
 import argparse
 import json
@@ -28,6 +33,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the tree may be read-only; nothing is cached in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 os.environ.setdefault("BOXOBAN_LEVELS", os.path.join(ROOT, "tests", "golden", "boxoban"))  # Sokoban (config 5) reads level files
@@ -261,7 +267,30 @@ class Harness:
         return self.max_ms(total * 1e3)
 
 
-def measure_config(hz, cfg_id, K, Wm, rank, cores, sample_clocks=False):
+DUMP_VIEWS = 256  # 256 views of RGBA as float32 are 38 MB: the dump stays under 64 MB with depth (9 MB) as well
+
+
+def dump_outputs(eng, out_dir, depth):
+    """what the device-resident step hands its caller, after its last step, as float32 / float64 .npy files: the rewards of every
+    agent, the done flags of every env, and the RGBA (and depth) frames of a fixed, seeded sample of views (obs_views: their indices)
+    -- the whole obs tensor would take four times its 151 MB as float32"""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    views = np.sort(np.random.default_rng(0).choice(eng.N, min(eng.N, DUMP_VIEWS), replace=False))
+    idx = torch.from_numpy(views).cuda()
+
+    def dev(what):
+        return torch.as_tensor(eng.device_array(what), device="cuda")
+
+    out = {"rewards": dev("rewards").float(), "dones": dev("dones").float(), "obs": dev("obs")[idx].float(), "obs_views": views.astype(np.float64)}
+    if depth:
+        out["depth"] = dev("depth")[idx].float()
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy() if torch.is_tensor(a) else a)
+
+
+def measure_config(hz, cfg_id, K, Wm, rank, cores, sample_clocks=False, dump_dir=None):
     """one BASELINE single-GPU config on this rank's GPU: device-resident value, e2e through host buffers, roofline of the raster kernel"""
     from megaverse_b200 import capi, sharding
 
@@ -296,22 +325,23 @@ def measure_config(hz, cfg_id, K, Wm, rank, cores, sample_clocks=False):
     l0 = eng.kernel_launches()
     ms = hz.timed_flushed(stream, eng.sync, dev_step, K, Wm)
     launches = eng.kernel_launches() - l0
+    if dump_dir:
+        dump_outputs(eng, dump_dir, depth)
     ms_warm = hz.timed(stream, dev_step, K, Wm)
     eng.sync()
     clocks = sampler.stop() if sampler else None
 
     # ---- end-to-end through host buffers
-    Ke = max(20, min(K, 200))
     for t in range(3):
         host_step(t)
-    ms_e = hz.timed_host_flushed(stream, host_step, Ke, Wm)
-    ms_e_warm = hz.timed(stream, host_step, Ke, Wm)
+    ms_e = hz.timed_host_flushed(stream, host_step, K, Wm)
+    ms_e_warm = hz.timed(stream, host_step, K, Wm)
 
     # ---- roofline of the dominant kernel (rasteriser): CUDA events around the kernel on the engine stream, L2 flushed before
     peak, peak_src = measured_peaks()
     eng.set_option("overlap", 0)  # kernels back to back so that each can be timed on its own
     ras, stp = [], []
-    for t in range(24):
+    for t in range(4 + K):  # the first 4 are not counted
         with torch.cuda.stream(stream):
             hz.flush.zero_()
         dev_step(Wm + t)
@@ -330,8 +360,8 @@ def measure_config(hz, cfg_id, K, Wm, rank, cores, sample_clocks=False):
     eng.close()
     return {"workload": cfg["name"] + " per GPU, random one-bit actions, resets included",
             "value": N * world * K / (ms / 1e3), "ms_per_step": ms / K, "value_l2_warm": N * world * K / (ms_warm / 1e3), "ms_per_step_l2_warm": ms_warm / K,
-            "e2e": {"value": N * world * Ke / (ms_e / 1e3), "unit": UNIT, "h2d_bytes_per_step": N * 4, "d2h_bytes_per_step": obs_bytes + N * 8 + E, "steps": Ke,
-                    "ms_per_step": ms_e / Ke, "value_l2_warm": N * world * Ke / (ms_e_warm / 1e3), "d2h_gbs": obs_bytes / (ms_e / Ke / 1e3) / 1e9},
+            "e2e": {"value": N * world * K / (ms_e / 1e3), "unit": UNIT, "h2d_bytes_per_step": N * 4, "d2h_bytes_per_step": obs_bytes + N * 8 + E, "steps": K,
+                    "ms_per_step": ms_e / K, "value_l2_warm": N * world * K / (ms_e_warm / 1e3), "d2h_gbs": obs_bytes / (ms_e / K / 1e3) / 1e9},
             "roofline": roofline, "gpu_launches": int(launches), "faults": int(faults), "clocks": clocks, "raster": rcfg, "views_per_gpu": N}
 
 
@@ -444,6 +474,7 @@ def main():
     ap.add_argument("--config", type=int, default=HEADLINE, choices=sorted(CONFIGS), help="BASELINE config to headline (default: the largest)")
     ap.add_argument("--only-headline", action="store_true", help="skip the other configs' sub-records")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the headline's outputs of its last timed step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
     rank, local_rank, world = dist_env()
     K, Wm = args.steps, max(args.warmup, 3)
@@ -471,9 +502,7 @@ def main():
 
     import torch
     import torch.distributed as dist
-    from megaverse_b200 import _build
 
-    _build.build_all()
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device (the product has no CPU fallback)")
     torch.cuda.set_device(local_rank)
@@ -482,7 +511,7 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     hz = Harness(torch, dist, world, local_rank)
 
-    main_rec = measure_config(hz, args.config, K, Wm, rank, cores, sample_clocks=True)
+    main_rec = measure_config(hz, args.config, K, Wm, rank, cores, sample_clocks=True, dump_dir=args.dump_outputs if rank == 0 else None)
     others = {}
     if world == 1 and not args.only_headline:
         for cid in sorted(CONFIGS):
