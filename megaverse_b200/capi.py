@@ -234,7 +234,8 @@ class Engine:
         out = (C.c_ulonglong * 16)()
         lib().mv_debug_raster_stats.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
         self._ck(lib().mv_debug_raster_stats(self._h, out if read else None, 1 if enable else 0))
-        names = ["work_items", "instances", "visible_instances", "items", "clipped_items", "triangles", "batches", "sub_passes", "cyc_head", "cyc_tma_wait", "cyc_instance", "cyc_item", "cyc_tile", "cyc_total"]
+        names = ["work_items", "instances", "visible_instances", "items", "clipped_items", "triangles", "batches", "sub_passes", "cyc_head", "cyc_tma_wait", "cyc_instance", "cyc_item", "cyc_tile", "cyc_total",
+                 "pairs_evaluated", "pairs_in_boxes"]  # (tile, triangle) pairs: kept by the binning / in the triangles' pixel boxes
         return {n: int(out[i]) for i, n in enumerate(names)}
 
     def last_kernel_ms(self):

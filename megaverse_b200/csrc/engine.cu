@@ -392,6 +392,7 @@ struct mv_engine {
     // work counter advances by items + grid per launch and the host keeps the base instead of resetting the counter (no memset node
     // between the step kernel and its programmatic dependent).
     int launchView(mvr::ViewParams &vp, int grid, bool dependent) {
+        if ((vp.W / 32) * (vp.bandRows / 4) > mvr::kMaxBandTiles) { setError("raster band has more tiles than the bins hold"); return MV_ERR_ARG; }
         vp.workCounter = d_workCounter.p; vp.counterBase = counterBase;
         counterBase += uint32_t(vp.N) * uint32_t(vp.bands) + uint32_t(grid);
         cudaLaunchConfig_t cfg = {};
@@ -730,7 +731,7 @@ int mv_create(const char *scenario, int w, int h, int num_envs, int num_agents, 
     *out = nullptr;
     const int sc = scenario ? mv::scenarioFromName(scenario) : -1;
     if (sc < 0) { g_createError = std::string("unknown scenario ") + (scenario ? scenario : "(null)"); return MV_ERR_ARG; }
-    if (w <= 0 || h <= 0 || w % 32 != 0 || h % 4 != 0 || (w / 32) * (h / 4) > 128) { g_createError = "render size must be a multiple of 32x4 with at most 128 tiles"; return MV_ERR_ARG; }
+    if (w <= 0 || h <= 0 || w % 32 != 0 || h % 4 != 0 || (w / 32) * (h / 4) > mvr::kMaxBandTiles) { g_createError = "render size must be a multiple of 32x4 with at most 128 tiles"; return MV_ERR_ARG; }
     if (num_envs <= 0 || num_agents <= 0 || num_agents > MV_MAX_AGENTS) { g_createError = "bad num_envs / num_agents_per_env"; return MV_ERR_ARG; }
     for (int i = 0; i < nparams; ++i) {
         if (!keys || !keys[i] || !vals) { g_createError = "null parameter key / value array"; return MV_ERR_ARG; }
@@ -1175,7 +1176,8 @@ int mv_faults(mv_handle h, int32_t *out) {
     *out = f;
     return MV_OK;
 }
-// totals since enable: {work items, instances read, instances with visible items, items, clipped items, triangles, batches, -}
+// totals since enable: {work items, instances read, instances with visible items, items, clipped items, triangles, batches, item
+// sub-passes, six thread-0 cycle counts, (tile, triangle) pairs kept by the binning, pairs in the triangles' pixel boxes}
 int mv_debug_raster_stats(mv_handle h, unsigned long long *out16, int enable) {
     if (!h) return MV_ERR_ARG;
     DeviceGuard dg__(h->device);
@@ -1373,7 +1375,7 @@ int mv_debug_get_view(mv_handle h, int env, int agent, float *out16) {
 }
 
 int mv_debug_render_instances(const float *view16, const float *inst18, int n, int w, int h, uint8_t *rgba, float *depth) {
-    if (!view16 || !inst18 || n < 0 || n > 4096 || w % 32 || h % 4 || (w / 32) * (h / 4) > 128) return MV_ERR_ARG;
+    if (!view16 || !inst18 || n < 0 || n > 4096 || w % 32 || h % 4 || (w / 32) * (h / 4) > mvr::kMaxBandTiles) return MV_ERR_ARG;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return MV_ERR_CUDA;
     // instances must arrive boxes-first (draw order); count the leading boxes

@@ -11,10 +11,11 @@
 //     3. item pass, one thread per (visible box face | mesh triangle): object-space back-face test of mesh triangles, vertices,
 //        near/far clip, projection, 8-bit sub-pixel
 //        snap, integer edge set-up with the top-left rule folded into the constants -> TriCover / TriShade records appended
-//        to the CTA's triangle list IN SHARED MEMORY (no global scratch, no bins, no global atomics)
-//     4. tile pass, warps pull 32x4-pixel tiles of the band from a shared-memory counter: lanes scan the list's pixel boxes
-//        32 at a time; triangles of at most kSmallArea pixels in the tile are evaluated one lane per triangle (packed 64-bit
-//        shared-memory atomicMax), the others by the whole warp (lane = 4 adjacent pixels, best fragment in registers); exact integer edge functions,
+//        to the CTA's triangle list IN SHARED MEMORY (no global scratch, no global atomics)
+//     4. binning, once per batch, all threads: every (tile, triangle) pair of a triangle's pixel box is tested edge by edge against
+//        the tile's samples (exact integers, conservative) -> one bit per list entry in the tile's bin (shared memory)
+//     5. tile pass, warps pull 32x4-pixel tiles of the band from a shared-memory counter and walk the tile's bin in list order: the
+//        whole warp evaluates each triangle (lane = 4 adjacent pixels, best fragment in registers); exact integer edge functions,
 //        nearest depth wins, later draw wins ties (LESS_OR_EQUAL); the single winner per pixel is shaded (deferred) and
 //        each lane stores its 4 pixels with one 128-bit store -- 8 lanes cover one full 128-byte line of the obs tensor
 //   A view with more triangles than the list holds is drawn in several batches: the per-pixel best fragment of earlier
@@ -69,11 +70,8 @@ constexpr int kInstChunk = MV_VIEW_INST_CHUNK;   // instances per TMA chunk (one
 static_assert(kInstChunk <= kThreads && kInstChunk <= 128, "one thread per instance of a chunk; slow-list entries keep 7 bits of it");
 constexpr int kXfWords = 23;      // per instance: model-view (12: three rows of each column), normal matrix (9), colour, mesh | face mask << 8
 constexpr int kClipVerts = 6;     // a triangle clipped by two planes has at most 5 vertices
-constexpr int kSmallList = 128;   // small triangles of a tile collected before they are evaluated (32 at a time, one lane each)
-#ifndef MV_SMALL_AREA
-#define MV_SMALL_AREA 4
-#endif
-constexpr int kSmallArea = MV_SMALL_AREA;    // triangles covering at most this many pixels of a tile are evaluated by one lane (swept 0..64: profiles/r2e_summary.txt)
+constexpr int kMaxBandTiles = 128;  // 32x4 tiles of one (view, band) work item (the host keeps to it)
+constexpr uint32_t kSmemOptin = 232448u;  // shared memory one CTA may opt in to on sm_100 (227 KB)
 // a fragment is (~depth bits << 32) | (draw-order key << kIdxBits) | index in the CTA's triangle list
 constexpr int kIdxBits = 10;
 constexpr uint32_t kStaleIdx = (1u << kIdxBits) - 1u;  // "already shaded in an earlier batch"
@@ -100,8 +98,9 @@ struct ViewParams {
     const uint32_t *ready;       // [E] step-kernel completion stamps (nullptr: plain stream order)
     uint32_t readyStamp;         // value ready[env] holds once this step's state, instances and views of env are written
     uint32_t *consumed;          // optional [E]: += 1 when a work item of env has read the env's instance list and view (step/raster overlap)
-    unsigned long long *stats;   // optional [16]: work items, instances, visible instances, items, clipped items, triangles, batches, -, then
-                                 // thread-0 cycles: head (claim, stamp, view), TMA waits, instance passes, item passes, final tile pass, whole item
+    unsigned long long *stats;   // optional [16]: work items, instances, visible instances, items, clipped items, triangles, batches, item
+                                 // sub-passes, then thread-0 cycles: head (claim, stamp, view), TMA waits, instance passes, item passes, final
+                                 // binning + tile pass, whole item; then (tile, triangle) pairs: kept by the binning (evaluated), in the pixel boxes
     unsigned long long *spill;   // [gridDim.x][spillStride] per-CTA fragment slab for views drawn in several batches
     int spillStride;             // >= W * bandRows
     // cost-ordered work queue (optional; viewBase == 0, N = E * A): claim c draws item c % (A * bands) of env order[c / (A * bands)].  Every
@@ -124,22 +123,24 @@ struct ViewParams {
     float p00, p11, p22, p32;
 };
 
-struct SmemLayout { uint32_t stage, cover, shade, xf, off, frag, small, meshV, meshI, clip, slow, sched, misc, total; };
+struct SmemLayout { uint32_t stage, cover, shade, xf, off, meshV, meshI, slow, sched, misc, bins, clip, binTiles, total; };
 struct ViewMisc {
     float view[16];
     int32_t counts[8];
     int32_t nTris;      // append counter of the current batch (may run past triCap: the excess is retried in the next batch)
     int32_t nValid;     // first refused list index of the current batch (INT_MAX: none)
-    int32_t tileCtr;
+    int32_t tileCtr;    // next tile of the band (binTris sets it to the first tile of its round)
     uint32_t claim;     // this work item; claimed (and, when its env was ready, its view / counts / first chunk fetched) during the previous tile pass
     int32_t prefetched;
     int32_t lastCta;    // cost-ordered queue: this CTA is the last one to leave the grid (it sorts the views for the next launch)
     int32_t wsum[kWarps];
     int32_t nSlow[2];   // entries of the two slow-item lists (alternating per item sub-pass)
-    uint32_t stat[8];   // debug counters of the current work item ([7]: item sub-passes)
+    uint32_t stat[10];  // debug counters of the current work item (stats slots 0..7, then 14, 15)
     alignas(8) unsigned long long bar[2];
     unsigned long long itemStart;  // clock64 when thread 0 started the current work item (after the wait for its env)
 };
+// per-tile bins: one bit per list entry, `binWords` words per tile
+__host__ __device__ inline int binWords(int triCap) { return (triCap + 31) >> 5; }
 __host__ __device__ inline SmemLayout smemLayout(int triCap) {
     SmemLayout L;
     uint32_t o = 0;
@@ -148,16 +149,23 @@ __host__ __device__ inline SmemLayout smemLayout(int triCap) {
     L.shade = o; o += uint32_t(triCap) * uint32_t(sizeof(TriShade));
     L.xf = o; o += uint32_t(kXfWords) * kInstChunk * 4u;
     L.off = o; o += (kInstChunk + 4u) * 4u;
-    // per warp: 128 fragments (tile pass) -- the same bytes hold the warp's clip polygons during the item pass (4 x kClipVerts x 40 B =
-    // 960 B <= 1024 B): neither keeps state across the other (fragments are zeroed per tile, polygons rebuilt per clipped item)
-    L.frag = o; o += uint32_t(kWarps) * 128u * 8u;
     L.meshV = o; o += uint32_t(kMeshVerts) * 6u * 4u;
     L.meshI = o; o += (uint32_t(kMeshIdx) + 15u) & ~15u;
-    L.clip = L.frag;
-    L.small = o; o += uint32_t(kWarps) * kSmallList * 2u;       // per warp: list indices of the small triangles of the current tile
     L.slow = o; o += 2u * kThreads * 2u;                        // two lists of at most one entry per thread
     L.sched = o; o += 256u * 4u;                                // cost classes of the counting sort (last CTA of a cost-ordered launch)
     L.misc = o; o += (uint32_t(sizeof(ViewMisc)) + 15u) & ~15u;
+    // the tile bins of the current batch (binning + tile pass) -- the same bytes hold the warps' clip polygons during the item pass (per
+    // warp 4 x kClipVerts x 40 B = 960 B <= 1024 B): neither keeps state across the other (the bins are rebuilt per batch once the item
+    // pass has finished the list, the polygons per clipped item).  Bins for kMaxBandTiles tiles where shared memory allows (up to
+    // tri_cap 640 that is no more than the clip polygons take); at the largest lists only what fits, and the tile pass then bins and
+    // draws a band in several rounds of binTiles tiles.
+    const uint32_t clipBytes = uint32_t(kWarps) * 1024u, tileBytes = uint32_t(binWords(triCap)) * 4u;
+    uint32_t binBytes = uint32_t(kMaxBandTiles) * tileBytes;
+    if (o + binBytes > kSmemOptin) binBytes = o + clipBytes < kSmemOptin ? (kSmemOptin - o) / tileBytes * tileBytes : 0u;
+    binBytes = binBytes > clipBytes ? binBytes : clipBytes;
+    L.bins = o; o += binBytes;
+    L.clip = L.bins;
+    L.binTiles = binBytes / tileBytes;
     L.total = o;
     return L;
 }
@@ -557,223 +565,14 @@ __device__ __forceinline__ unsigned long long packFrag(float z, uint32_t key, in
     return ((unsigned long long)(~asc) << 32) | (unsigned long long)((key << kIdxBits) | uint32_t(idx));
 }
 
-// All tiles of the band against the current batch of `count` triangles.  batch 0 paints every pixel (background included); later
-// batches repaint only the pixels they win.  Unless `final`, the per-pixel best fragment is parked in the CTA's spill slab with its
-// list index replaced by kStaleIdx (the list is about to be overwritten).
-// out of line on purpose: the tile pass is called from two places (a full triangle list in mid-view, the end of the view) and two inlined
-// copies of it pushed the kernel's hot code out of the instruction cache (Collect 1024 x 4: 2.65 ms inlined, 1.70 ms called)
+// Out of line on purpose: the tile pass (with the binning) is called from two places (a full triangle list in mid-view, the end of the
+// view) and two inlined copies of it pushed the kernel's hot code out of the instruction cache (Collect 1024 x 4: 2.65 ms inlined, 1.70 ms called)
 #ifdef MV_TILE_FORCEINLINE
 #define MV_TILE_INLINE __forceinline__
 #else
 #define MV_TILE_INLINE __noinline__
 #endif
 extern __shared__ __align__(128) unsigned char g_viewSmem[];  // the CTA's dynamic shared memory (carved up by smemLayout)
-
-template <bool FAST>
-__device__ MV_TILE_INLINE void tilePass(const ViewParams &P, int count, unsigned long long *spill, int view, int rowLo, int bandTiles, int batch, bool final) {
-    // addresses derived from the shared-memory symbol itself, so that this out-of-line function keeps shared-space loads and atomics
-    const SmemLayout L = smemLayout(P.triCap);
-    const TriCover *cover = reinterpret_cast<const TriCover *>(g_viewSmem + L.cover);
-    const TriShade *shade = reinterpret_cast<const TriShade *>(g_viewSmem + L.shade);
-    unsigned long long *frag = reinterpret_cast<unsigned long long *>(g_viewSmem + L.frag) + (threadIdx.x >> 5) * 128;
-    uint16_t *smallList = reinterpret_cast<uint16_t *>(g_viewSmem + L.small) + (threadIdx.x >> 5) * kSmallList;
-    int32_t *tileCtr = &reinterpret_cast<ViewMisc *>(g_viewSmem + L.misc)->tileCtr;
-    const int lane = threadIdx.x & 31;
-    const int tilesX = P.W >> 5;
-    for (;;) {
-        int tile = 0;
-        if (lane == 0) tile = atomicAdd(tileCtr, 1);
-        tile = __shfl_sync(0xffffffffu, tile, 0);
-        if (tile >= bandTiles) break;
-        const int tk = tile / tilesX, ty = tk;  // (drawing the tile rows from the middle outwards -- horizon first, sky and floor last -- was measured: no effect)
-        const int tx0 = (tile - tk * tilesX) * 32, ty0 = rowLo + ty * 4;
-        const int px = tx0 + (lane & 7) * 4, py = ty0 + (lane >> 3);
-        const int sx32 = px * 256 + 128, sy32 = py * 256 + 128;
-        unsigned long long best[4] = {0ull, 0ull, 0ull, 0ull};
-#pragma unroll
-        for (int k = 0; k < 4; ++k) frag[lane * 4 + k] = 0ull;
-        __syncwarp();
-
-        // Small triangles (at most kSmallArea pixels of the tile) are evaluated one lane per triangle; they are first COLLECTED over the
-        // whole list scan and then evaluated 32 at a time -- scattered over the scan they would cost a serial pixel walk per 32 list
-        // entries with one or two lanes busy.
-        int nSmall = 0;
-        auto evalSmall = [&](int n) {
-            __syncwarp();
-            for (int s0 = 0; s0 < n; s0 += 32) {
-                if (s0 + lane < n) {
-                    const int j = int(smallList[s0 + lane]);
-                    const uint2 bb = *reinterpret_cast<const uint2 *>(&cover[j].bx);
-                    const int bx0 = max(int(bb.x & 0xffffu), tx0), bx1 = min(int(bb.x >> 16), tx0 + 31);
-                    const int by0 = max(int(bb.y & 0xffffu), ty0), by1 = min(int(bb.y >> 16), ty0 + 3);
-                    const EdgeEval e = loadCover(cover + j);
-                    for (int y = by0; y <= by1; ++y) {
-                        const int sy = y * 256 + 128, sx0 = bx0 * 256 + 128;
-                        if (e.small) {
-                            int F0 = int(e.C0) + e.A0 * sx0 + e.B0 * sy, F1 = int(e.C1) + e.A1 * sx0 + e.B1 * sy, F2 = int(e.C2) + e.A2 * sx0 + e.B2 * sy;
-                            for (int x = bx0; x <= bx1; ++x) {
-                                if ((F0 | F1 | F2) >= 0) {
-                                    const float l0 = float(F0 + e.u0) * e.invArea, l1 = float(F1 + e.u1) * e.invArea, l2 = float(F2 + e.u2) * e.invArea;
-                                    const float z = (l0 * e.z0 + l1 * e.z1) + l2 * e.z2;
-                                    if (z <= 1.0f) atomicMax(&frag[(y - ty0) * 32 + (x - tx0)], packFrag(z, e.key, j));
-                                }
-                                F0 += e.A0 * 256; F1 += e.A1 * 256; F2 += e.A2 * 256;
-                            }
-                        } else {
-                            long long F0 = e.C0 + (long long)e.A0 * sx0 + (long long)e.B0 * sy, F1 = e.C1 + (long long)e.A1 * sx0 + (long long)e.B1 * sy,
-                                      F2 = e.C2 + (long long)e.A2 * sx0 + (long long)e.B2 * sy;
-                            for (int x = bx0; x <= bx1; ++x) {
-                                if ((F0 | F1 | F2) >= 0) {
-                                    const float l0 = float(F0 + e.u0) * e.invArea, l1 = float(F1 + e.u1) * e.invArea, l2 = float(F2 + e.u2) * e.invArea;
-                                    const float z = (l0 * e.z0 + l1 * e.z1) + l2 * e.z2;
-                                    if (z <= 1.0f) atomicMax(&frag[(y - ty0) * 32 + (x - tx0)], packFrag(z, e.key, j));
-                                }
-                                F0 += (long long)e.A0 * 256; F1 += (long long)e.A1 * 256; F2 += (long long)e.A2 * 256;
-                            }
-                        }
-                    }
-                }
-            }
-            __syncwarp();
-        };
-        int base = 0;
-        do {  // (one call site of evalSmall: the scan pauses when the list could overflow)
-        nSmall = 0;
-        for (; base < count && nSmall + 32 <= kSmallList; base += 32) {
-            const int j = base + lane;
-            bool ov = false, small = false;
-            if (j < count) {
-                const uint2 bb = *reinterpret_cast<const uint2 *>(&cover[j].bx);
-                const int bx0 = max(int(bb.x & 0xffffu), tx0), bx1 = min(int(bb.x >> 16), tx0 + 31);
-                const int by0 = max(int(bb.y & 0xffffu), ty0), by1 = min(int(bb.y >> 16), ty0 + 3);
-                ov = bx0 <= bx1 && by0 <= by1;
-                small = ov && (bx1 - bx0 + 1) * (by1 - by0 + 1) <= kSmallArea;
-            }
-            {
-                const unsigned sm = __ballot_sync(0xffffffffu, small);
-                if (sm) {
-                    if (small) smallList[nSmall + __popc(sm & ((1u << lane) - 1u))] = uint16_t(j);
-                    nSmall += __popc(sm);
-                }
-            }
-            // ---- larger triangles: whole warp, lane = 4 pixels, the record is broadcast from shared memory
-            unsigned bits = __ballot_sync(0xffffffffu, ov && !small);
-            while (bits) {
-                const int bsel = __ffs(bits) - 1;
-                bits &= bits - 1;
-                const int ti = base + bsel;
-                const uint2 bb = *reinterpret_cast<const uint2 *>(&cover[ti].bx);
-                const int x0 = int(bb.x & 0xffffu), x1 = int(bb.x >> 16), y0 = int(bb.y & 0xffffu), y1 = int(bb.y >> 16);
-                if (px + 3 < x0 || px > x1 || py < y0 || py > y1) continue;
-                const EdgeEval e2 = loadCover(cover + ti);
-                if (e2.small) {
-                    int F0 = int(e2.C0) + e2.A0 * sx32 + e2.B0 * sy32, F1 = int(e2.C1) + e2.A1 * sx32 + e2.B1 * sy32, F2 = int(e2.C2) + e2.A2 * sx32 + e2.B2 * sy32;
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) {
-                        if ((F0 | F1 | F2) >= 0) {
-                            const float l0 = float(F0 + e2.u0) * e2.invArea, l1 = float(F1 + e2.u1) * e2.invArea, l2 = float(F2 + e2.u2) * e2.invArea;
-                            const float z = (l0 * e2.z0 + l1 * e2.z1) + l2 * e2.z2;
-                            if (z <= 1.0f) { const unsigned long long f = packFrag(z, e2.key, ti); best[k] = f > best[k] ? f : best[k]; }
-                        }
-                        F0 += e2.A0 * 256; F1 += e2.A1 * 256; F2 += e2.A2 * 256;
-                    }
-                } else {
-                    long long F0 = e2.C0 + (long long)e2.A0 * sx32 + (long long)e2.B0 * sy32, F1 = e2.C1 + (long long)e2.A1 * sx32 + (long long)e2.B1 * sy32,
-                              F2 = e2.C2 + (long long)e2.A2 * sx32 + (long long)e2.B2 * sy32;
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) {
-                        if ((F0 | F1 | F2) >= 0) {
-                            const float l0 = float(F0 + e2.u0) * e2.invArea, l1 = float(F1 + e2.u1) * e2.invArea, l2 = float(F2 + e2.u2) * e2.invArea;
-                            const float z = (l0 * e2.z0 + l1 * e2.z1) + l2 * e2.z2;
-                            if (z <= 1.0f) { const unsigned long long f = packFrag(z, e2.key, ti); best[k] = f > best[k] ? f : best[k]; }
-                        }
-                        F0 += (long long)e2.A0 * 256; F1 += (long long)e2.A1 * 256; F2 += (long long)e2.A2 * 256;
-                    }
-                }
-            }
-        }
-        evalSmall(nSmall);
-        } while (base < count);
-        // ---- merge both paths (and the earlier batches), recompute the winner's barycentrics, shade, store
-        const int pixInTile = (lane >> 3) * 32 + (lane & 7) * 4;
-        unsigned long long *sp = spill + size_t(tile) * 128 + pixInTile;
-        unsigned long long f4[4];
-        if (batch > 0) {
-            const ulonglong2 s01 = *reinterpret_cast<const ulonglong2 *>(sp), s23 = *reinterpret_cast<const ulonglong2 *>(sp + 2);
-            f4[0] = s01.x; f4[1] = s01.y; f4[2] = s23.x; f4[3] = s23.y;
-        } else {
-            f4[0] = f4[1] = f4[2] = f4[3] = 0ull;
-        }
-        // winners of the lane's four pixels (list index, 0xffff = nothing new to shade), then ONE copy of the fragment stage in a rolled
-        // loop: the kernel's hot code has to stay inside the instruction cache (unrolled four times it did not)
-        unsigned long long winners = 0ull;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const unsigned long long fs = frag[pixInTile + k];
-            unsigned long long f = fs > best[k] ? fs : best[k];
-            f = f > f4[k] ? f : f4[k];
-            f4[k] = f;
-            const uint32_t ti = uint32_t(f) & kStaleIdx;
-            const bool fresh = f != 0ull && ti != kStaleIdx;
-            winners |= (unsigned long long)(fresh ? ti : 0xffffu) << (16 * k);
-        }
-        uint32_t o0 = 0xff000000u, o1 = 0xff000000u, o2 = 0xff000000u, o3 = 0xff000000u;
-        float w0 = 0.0f, w1 = 0.0f, w2 = 0.0f, w3 = 0.0f;
-        // (keeping the records of the previous pixel's triangle in registers across the iterations -- the lane's four pixels mostly belong
-        // to one triangle -- was measured: 20 % SLOWER, the loop then spills)
-#pragma unroll 1
-        for (int k = 0; k < 4; ++k) {
-            const uint32_t ti = uint32_t(winners >> (16 * k)) & 0xffffu;
-            if (ti == 0xffffu) continue;
-            const ShadeRec rec = loadShade(shade + ti);
-            const EdgeEval e = loadCover(cover + ti);
-            const int sx = sx32 + k * 256;
-            float l0, l1, l2;
-            if (e.small) {
-                l0 = float(int(e.C0) + e.A0 * sx + e.B0 * sy32 + e.u0) * e.invArea;
-                l1 = float(int(e.C1) + e.A1 * sx + e.B1 * sy32 + e.u1) * e.invArea;
-                l2 = float(int(e.C2) + e.A2 * sx + e.B2 * sy32 + e.u2) * e.invArea;
-            } else {
-                l0 = float(e.C0 + (long long)e.A0 * sx + (long long)e.B0 * sy32 + e.u0) * e.invArea;
-                l1 = float(e.C1 + (long long)e.A1 * sx + (long long)e.B1 * sy32 + e.u1) * e.invArea;
-                l2 = float(e.C2 + (long long)e.A2 * sx + (long long)e.B2 * sy32 + e.u2) * e.invArea;
-            }
-            float w;
-            const uint32_t c = shadePixel<FAST>(rec, l0, l1, l2, e.flat != 0, w);
-            if (k == 0) { o0 = c; w0 = w; } else if (k == 1) { o1 = c; w1 = w; } else if (k == 2) { o2 = c; w2 = w; } else { o3 = c; w3 = w; }
-        }
-        const bool fr0 = (winners & 0xffffull) != 0xffffull, fr1 = ((winners >> 16) & 0xffffull) != 0xffffull, fr2 = ((winners >> 32) & 0xffffull) != 0xffffull,
-                   fr3 = (winners >> 48) != 0xffffull;
-        uint8_t *obsPix = P.obs + ((size_t(view) * P.H + size_t(py)) * P.W + px) * 4;
-        float *depthPix = P.depth ? P.depth + (size_t(view) * P.H + size_t(py)) * P.W + px : nullptr;
-        if (batch == 0) {
-            *reinterpret_cast<uint4 *>(obsPix) = make_uint4(o0, o1, o2, o3);
-            if (depthPix) *reinterpret_cast<float4 *>(depthPix) = make_float4(w0, w1, w2, w3);
-        } else if (fr0 || fr1 || fr2 || fr3) {  // a later batch won some of this lane's pixels: this lane wrote the others itself, earlier
-            uint4 old = *reinterpret_cast<const uint4 *>(obsPix);
-            if (fr0) old.x = o0;
-            if (fr1) old.y = o1;
-            if (fr2) old.z = o2;
-            if (fr3) old.w = o3;
-            *reinterpret_cast<uint4 *>(obsPix) = old;
-            if (depthPix) {
-                float4 od = *reinterpret_cast<const float4 *>(depthPix);
-                if (fr0) od.x = w0;
-                if (fr1) od.y = w1;
-                if (fr2) od.z = w2;
-                if (fr3) od.w = w3;
-                *reinterpret_cast<float4 *>(depthPix) = od;
-            }
-        }
-        if (!final) {
-#pragma unroll
-            for (int k = 0; k < 4; ++k) f4[k] = f4[k] ? (f4[k] | (unsigned long long)kStaleIdx) : 0ull;
-            *reinterpret_cast<ulonglong2 *>(sp) = make_ulonglong2(f4[0], f4[1]);
-            *reinterpret_cast<ulonglong2 *>(sp + 2) = make_ulonglong2(f4[2], f4[3]);
-        }
-        __syncwarp();  // the warp's fragment buffer is cleared by the next tile
-    }
-}
 
 // ---------------------------------------------------------------------------------------------------- work queue
 // Next work item of the CTA (called by one thread): an index into [0, total), or >= total when the queue is empty.  Natural order: the
@@ -785,6 +584,259 @@ __device__ __forceinline__ uint32_t claimWork(const ViewParams &P, uint32_t tota
         return __ldcg(P.order + c / perEnv) * perEnv + c % perEnv;
     }
     return c;
+}
+
+// Claim the next work item now and, if its env's state is already published, fetch its view matrix, its counts and its first instance
+// chunk while this item's tiles are drawn (the stage buffers, M.view and M.counts are idle during the tile pass): the global round trips
+// of the item head then cost nothing.  One thread (thread 0, after the binning); its warp joins the tile pass a little later.
+__device__ __forceinline__ void claimNext(const ViewParams &P) {
+    const SmemLayout L = smemLayout(P.triCap);
+    MvInstance *stage = reinterpret_cast<MvInstance *>(g_viewSmem + L.stage);
+    ViewMisc &M = *reinterpret_cast<ViewMisc *>(g_viewSmem + L.misc);
+    const int bands = P.bands;
+    const uint32_t total = uint32_t(P.N) * uint32_t(bands);
+    const uint32_t nc = claimWork(P, total);
+    int pre = 0;
+    if (nc < total) {
+        const int nview = P.viewBase + int(nc / uint32_t(bands)), nenv = nview / P.A;
+        bool ready = true;
+        if (P.ready) {
+            uint32_t v;
+            asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(P.ready + nenv) : "memory");
+            ready = v == P.readyStamp;
+            if (ready) asm volatile("fence.proxy.async;" ::: "memory");
+        }
+        if (ready) {
+            float vm[16];
+            int32_t cn[8];
+#pragma unroll
+            for (int q = 0; q < 16; ++q) vm[q] = __ldcg(P.views + size_t(nview) * 16 + q);
+#pragma unroll
+            for (int q = 0; q < 8; ++q) cn[q] = __ldcg(P.instCounts + nenv * 8 + q);
+#pragma unroll
+            for (int q = 0; q < 16; ++q) M.view[q] = vm[q];
+#pragma unroll
+            for (int q = 0; q < 8; ++q) M.counts[q] = cn[q];
+            if (cn[1] > 0) {
+                const uint32_t bytes = uint32_t(min(cn[1], kInstChunk)) * uint32_t(sizeof(MvInstance));
+                mbarExpectTx(&M.bar[0], bytes);
+                bulkG2S(stage, P.instances + size_t(nenv) * size_t(P.instStride), bytes, &M.bar[0]);
+            }
+            pre = 1;
+        }
+    }
+    M.claim = nc; M.prefetched = pre;
+}
+
+// Bins of the current batch of `count` triangles for the band's tiles [t0, t1): bit j % 32 of bins[(tile - t0) * binWords + j / 32] is
+// set when list entry j may cover a sample of the tile.  Each (tile, triangle) pair of a triangle's pixel box is tested against the tile: every edge function at the
+// sample of (tile & box) where it is largest -- exact 64-bit integers, the top-left bias already in C -- and the pair is dropped only
+// when one edge is negative there, i.e. at every sample of the tile (a kept pair may still cover nothing; a covered sample is never
+// lost).  The pairs are spread over the lanes: a warp takes 32 list entries, scans their box tile counts and then tests one pair per
+// lane, so a floor triangle spanning the whole band does not hold up one thread.  Called by all threads, once the list is complete; also
+// points the tile counter at t0.
+__device__ __forceinline__ void binTris(const ViewParams &P, int count, int rowLo, int t0, int t1) {
+    const SmemLayout L = smemLayout(P.triCap);
+    const TriCover *cover = reinterpret_cast<const TriCover *>(g_viewSmem + L.cover);
+    uint32_t *bins = reinterpret_cast<uint32_t *>(g_viewSmem + L.bins);
+    ViewMisc &M = *reinterpret_cast<ViewMisc *>(g_viewSmem + L.misc);
+    const int words = binWords(P.triCap), tilesX = P.W >> 5, lane = threadIdx.x & 31;
+    for (int i = threadIdx.x; i < (t1 - t0) * words; i += kThreads) bins[i] = 0u;
+    if (threadIdx.x == 0) M.tileCtr = t0;
+    const int yLo = rowLo + (t0 / tilesX) * 4, yHi = rowLo + ((t1 - 1) / tilesX) * 4 + 3;  // the rows of [t0, t1)
+    __syncthreads();
+    uint32_t nBox = 0, nKept = 0;
+    for (int base = (threadIdx.x >> 5) * 32; base < count; base += kThreads) {
+        int n = 0;
+        if (base + lane < count) {
+            const uint2 bb = *reinterpret_cast<const uint2 *>(&cover[base + lane].bx);
+            const int y0 = max(int(bb.y & 0xffffu), yLo), y1 = min(int(bb.y >> 16), yHi);
+            if (y0 <= y1) n = ((int(bb.x >> 16) >> 5) - (int(bb.x & 0xffffu) >> 5) + 1) * (((y1 - rowLo) >> 2) - ((y0 - rowLo) >> 2) + 1);
+        }
+        int incl = n;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const int up = __shfl_up_sync(0xffffffffu, incl, d);
+            if (lane >= d) incl += up;
+        }
+        const int total = __shfl_sync(0xffffffffu, incl, 31);
+        for (int p0 = 0; p0 < total; p0 += 32) {
+            const int p = p0 + lane;
+            int o = 0;  // the entry pair p belongs to: the first lane whose inclusive count exceeds p
+#pragma unroll
+            for (int s = 16; s; s >>= 1)
+                if (__shfl_sync(0xffffffffu, incl, o + s - 1) <= p) o += s;
+            const int r = p - __shfl_sync(0xffffffffu, incl - n, o);
+            bool inRange = false, keep = false;
+            if (p < total) {
+                const TriCover *c = cover + base + o;
+                const uint2 bb = *reinterpret_cast<const uint2 *>(&c->bx);
+                const int x0 = int(bb.x & 0xffffu), x1 = int(bb.x >> 16);
+                const int y0 = max(int(bb.y & 0xffffu), yLo), y1 = min(int(bb.y >> 16), yHi);
+                const int ntx = (x1 >> 5) - (x0 >> 5) + 1, rq = r / ntx;
+                const int tx = (x0 >> 5) + (r - rq * ntx), ty = ((y0 - rowLo) >> 2) + rq, tile = ty * tilesX + tx;
+                inRange = tile >= t0 && tile < t1;  // (whole tile rows but the first and last of a round)
+                // sample centres of the tile inside the box, in 1/256 pixel
+                const long long sx0 = max(x0, tx * 32) * 256 + 128, sx1 = min(x1, tx * 32 + 31) * 256 + 128;
+                const long long sy0 = max(y0, rowLo + ty * 4) * 256 + 128, sy1 = min(y1, rowLo + ty * 4 + 3) * 256 + 128;
+                keep = inRange;
+#pragma unroll
+                for (int e = 0; e < 3; ++e) {
+                    const int A = c->A[e], B = c->B[e];
+                    keep = keep && c->C[e] + A * (A > 0 ? sx1 : sx0) + B * (B > 0 ? sy1 : sy0) >= 0;
+                }
+                if (keep) atomicOr(&bins[(tile - t0) * words + (base >> 5)], 1u << o);
+            }
+            nKept += uint32_t(__popc(__ballot_sync(0xffffffffu, keep)));
+            nBox += uint32_t(__popc(__ballot_sync(0xffffffffu, inRange)));
+        }
+    }
+    if (P.stats && lane == 0) { atomicAdd(&M.stat[8], nKept); atomicAdd(&M.stat[9], nBox); }
+    __syncthreads();
+}
+
+// All tiles of the band against the current batch of `count` triangles: the batch is binned first (all threads), then the warps draw
+// the tiles -- in one round unless the list is so long that shared memory holds the bins of fewer tiles than the band has.  batch 0
+// paints every pixel (background included); later batches repaint only the pixels they win.  Unless `final`, the per-pixel best
+// fragment is parked in the CTA's spill slab with its list index replaced by kStaleIdx (the list is about to be overwritten); if
+// `final`, thread 0 claims the next work item once the first round is binned.
+template <bool FAST>
+__device__ MV_TILE_INLINE void tilePass(const ViewParams &P, int count, unsigned long long *spill, int view, int rowLo, int bandTiles, int batch, bool final) {
+    // addresses derived from the shared-memory symbol itself, so that this out-of-line function keeps shared-space loads
+    const SmemLayout L = smemLayout(P.triCap);
+    const TriCover *cover = reinterpret_cast<const TriCover *>(g_viewSmem + L.cover);
+    const TriShade *shade = reinterpret_cast<const TriShade *>(g_viewSmem + L.shade);
+    const uint32_t *bins = reinterpret_cast<const uint32_t *>(g_viewSmem + L.bins);
+    int32_t *tileCtr = &reinterpret_cast<ViewMisc *>(g_viewSmem + L.misc)->tileCtr;
+    const int lane = threadIdx.x & 31;
+    const int tilesX = P.W >> 5, words = binWords(P.triCap), nWords = (count + 31) >> 5;
+    for (int t0 = 0; t0 < bandTiles; t0 += int(L.binTiles)) {
+        const int t1 = min(bandTiles, t0 + int(L.binTiles));
+        if (t0) __syncthreads();  // the previous round's bins and tile counter are no longer read
+        binTris(P, count, rowLo, t0, t1);
+        if (final && t0 == 0 && threadIdx.x == 0) claimNext(P);
+        for (;;) {
+            int tile = 0;
+            if (lane == 0) tile = atomicAdd(tileCtr, 1);
+            tile = __shfl_sync(0xffffffffu, tile, 0);
+            if (tile >= t1) break;
+            const int tk = tile / tilesX, ty = tk;  // (drawing the tile rows from the middle outwards -- horizon first, sky and floor last -- was measured: no effect)
+            const int tx0 = (tile - tk * tilesX) * 32, ty0 = rowLo + ty * 4;
+            const int px = tx0 + (lane & 7) * 4, py = ty0 + (lane >> 3);
+            const int sx32 = px * 256 + 128, sy32 = py * 256 + 128;
+            unsigned long long best[4] = {0ull, 0ull, 0ull, 0ull};
+            // the tile's triangles in list order (the result does not depend on it: a max), whole warp, lane = 4 pixels, the record is
+            // broadcast from shared memory
+            const uint32_t *bin = bins + (tile - t0) * words;
+            for (int w = 0; w < nWords; ++w) {
+                unsigned bits = bin[w];
+                while (bits) {
+                    const int ti = w * 32 + __ffs(bits) - 1;
+                    bits &= bits - 1;
+                    const EdgeEval e2 = loadCover(cover + ti);
+                    if (e2.small) {
+                        int F0 = int(e2.C0) + e2.A0 * sx32 + e2.B0 * sy32, F1 = int(e2.C1) + e2.A1 * sx32 + e2.B1 * sy32, F2 = int(e2.C2) + e2.A2 * sx32 + e2.B2 * sy32;
+#pragma unroll
+                        for (int k = 0; k < 4; ++k) {
+                            if ((F0 | F1 | F2) >= 0) {
+                                const float l0 = float(F0 + e2.u0) * e2.invArea, l1 = float(F1 + e2.u1) * e2.invArea, l2 = float(F2 + e2.u2) * e2.invArea;
+                                const float z = (l0 * e2.z0 + l1 * e2.z1) + l2 * e2.z2;
+                                if (z <= 1.0f) { const unsigned long long f = packFrag(z, e2.key, ti); best[k] = f > best[k] ? f : best[k]; }
+                            }
+                            F0 += e2.A0 * 256; F1 += e2.A1 * 256; F2 += e2.A2 * 256;
+                        }
+                    } else {
+                        long long F0 = e2.C0 + (long long)e2.A0 * sx32 + (long long)e2.B0 * sy32, F1 = e2.C1 + (long long)e2.A1 * sx32 + (long long)e2.B1 * sy32,
+                                  F2 = e2.C2 + (long long)e2.A2 * sx32 + (long long)e2.B2 * sy32;
+#pragma unroll
+                        for (int k = 0; k < 4; ++k) {
+                            if ((F0 | F1 | F2) >= 0) {
+                                const float l0 = float(F0 + e2.u0) * e2.invArea, l1 = float(F1 + e2.u1) * e2.invArea, l2 = float(F2 + e2.u2) * e2.invArea;
+                                const float z = (l0 * e2.z0 + l1 * e2.z1) + l2 * e2.z2;
+                                if (z <= 1.0f) { const unsigned long long f = packFrag(z, e2.key, ti); best[k] = f > best[k] ? f : best[k]; }
+                            }
+                            F0 += (long long)e2.A0 * 256; F1 += (long long)e2.A1 * 256; F2 += (long long)e2.A2 * 256;
+                        }
+                    }
+                }
+            }
+            // ---- merge with the earlier batches, recompute the winner's barycentrics, shade, store
+            const int pixInTile = (lane >> 3) * 32 + (lane & 7) * 4;
+            unsigned long long *sp = spill + size_t(tile) * 128 + pixInTile;
+            unsigned long long f4[4];
+            if (batch > 0) {
+                const ulonglong2 s01 = *reinterpret_cast<const ulonglong2 *>(sp), s23 = *reinterpret_cast<const ulonglong2 *>(sp + 2);
+                f4[0] = s01.x; f4[1] = s01.y; f4[2] = s23.x; f4[3] = s23.y;
+            } else {
+                f4[0] = f4[1] = f4[2] = f4[3] = 0ull;
+            }
+            // winners of the lane's four pixels (list index, 0xffff = nothing new to shade), then ONE copy of the fragment stage in a rolled
+            // loop: the kernel's hot code has to stay inside the instruction cache (unrolled four times it did not)
+            unsigned long long winners = 0ull;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const unsigned long long f = best[k] > f4[k] ? best[k] : f4[k];
+                f4[k] = f;
+                const uint32_t ti = uint32_t(f) & kStaleIdx;
+                const bool fresh = f != 0ull && ti != kStaleIdx;
+                winners |= (unsigned long long)(fresh ? ti : 0xffffu) << (16 * k);
+            }
+            uint32_t o0 = 0xff000000u, o1 = 0xff000000u, o2 = 0xff000000u, o3 = 0xff000000u;
+            float w0 = 0.0f, w1 = 0.0f, w2 = 0.0f, w3 = 0.0f;
+            // (keeping the records of the previous pixel's triangle in registers across the iterations -- the lane's four pixels mostly belong
+            // to one triangle -- was measured: 20 % SLOWER, the loop then spills)
+#pragma unroll 1
+            for (int k = 0; k < 4; ++k) {
+                const uint32_t ti = uint32_t(winners >> (16 * k)) & 0xffffu;
+                if (ti == 0xffffu) continue;
+                const ShadeRec rec = loadShade(shade + ti);
+                const EdgeEval e = loadCover(cover + ti);
+                const int sx = sx32 + k * 256;
+                float l0, l1, l2;
+                if (e.small) {
+                    l0 = float(int(e.C0) + e.A0 * sx + e.B0 * sy32 + e.u0) * e.invArea;
+                    l1 = float(int(e.C1) + e.A1 * sx + e.B1 * sy32 + e.u1) * e.invArea;
+                    l2 = float(int(e.C2) + e.A2 * sx + e.B2 * sy32 + e.u2) * e.invArea;
+                } else {
+                    l0 = float(e.C0 + (long long)e.A0 * sx + (long long)e.B0 * sy32 + e.u0) * e.invArea;
+                    l1 = float(e.C1 + (long long)e.A1 * sx + (long long)e.B1 * sy32 + e.u1) * e.invArea;
+                    l2 = float(e.C2 + (long long)e.A2 * sx + (long long)e.B2 * sy32 + e.u2) * e.invArea;
+                }
+                float w;
+                const uint32_t c = shadePixel<FAST>(rec, l0, l1, l2, e.flat != 0, w);
+                if (k == 0) { o0 = c; w0 = w; } else if (k == 1) { o1 = c; w1 = w; } else if (k == 2) { o2 = c; w2 = w; } else { o3 = c; w3 = w; }
+            }
+            const bool fr0 = (winners & 0xffffull) != 0xffffull, fr1 = ((winners >> 16) & 0xffffull) != 0xffffull, fr2 = ((winners >> 32) & 0xffffull) != 0xffffull,
+                       fr3 = (winners >> 48) != 0xffffull;
+            uint8_t *obsPix = P.obs + ((size_t(view) * P.H + size_t(py)) * P.W + px) * 4;
+            float *depthPix = P.depth ? P.depth + (size_t(view) * P.H + size_t(py)) * P.W + px : nullptr;
+            if (batch == 0) {
+                *reinterpret_cast<uint4 *>(obsPix) = make_uint4(o0, o1, o2, o3);
+                if (depthPix) *reinterpret_cast<float4 *>(depthPix) = make_float4(w0, w1, w2, w3);
+            } else if (fr0 || fr1 || fr2 || fr3) {  // a later batch won some of this lane's pixels: this lane wrote the others itself, earlier
+                uint4 old = *reinterpret_cast<const uint4 *>(obsPix);
+                if (fr0) old.x = o0;
+                if (fr1) old.y = o1;
+                if (fr2) old.z = o2;
+                if (fr3) old.w = o3;
+                *reinterpret_cast<uint4 *>(obsPix) = old;
+                if (depthPix) {
+                    float4 od = *reinterpret_cast<const float4 *>(depthPix);
+                    if (fr0) od.x = w0;
+                    if (fr1) od.y = w1;
+                    if (fr2) od.z = w2;
+                    if (fr3) od.w = w3;
+                    *reinterpret_cast<float4 *>(depthPix) = od;
+                }
+            }
+            if (!final) {
+#pragma unroll
+                for (int k = 0; k < 4; ++k) f4[k] = f4[k] ? (f4[k] | (unsigned long long)kStaleIdx) : 0ull;
+                *reinterpret_cast<ulonglong2 *>(sp) = make_ulonglong2(f4[0], f4[1]);
+                *reinterpret_cast<ulonglong2 *>(sp + 2) = make_ulonglong2(f4[2], f4[3]);
+            }
+        }
+    }
 }
 
 // ---------------------------------------------------------------------------------------------------- the kernel
@@ -805,7 +857,7 @@ template <bool FAST> __global__ void MV_VIEW_BOUNDS viewKernel(const __grid_cons
     uint8_t *meshI = smem + L.meshI;
     uint16_t *slowAll = reinterpret_cast<uint16_t *>(smem + L.slow);  // [2][kThreads]: instance-in-chunk | item << 7 | done << 15
     ClipVert *clipScratch = reinterpret_cast<ClipVert *>(smem + L.clip + (threadIdx.x >> 5) * 1024u);
-    static_assert(4 * kClipVerts * sizeof(ClipVert) <= 1024, "a warp's clip polygons share its fragment buffer");
+    static_assert(4 * kClipVerts * sizeof(ClipVert) <= 1024, "a warp's clip polygons fit its 1 KB of the bin region");
     ViewMisc &M = *reinterpret_cast<ViewMisc *>(smem + L.misc);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 
@@ -869,9 +921,8 @@ template <bool FAST> __global__ void MV_VIEW_BOUNDS viewKernel(const __grid_cons
             M.itemStart = (unsigned long long)clock64();
             M.nTris = 0;
             M.nValid = 0x7fffffff;
-            M.tileCtr = 0;
             M.nSlow[0] = 0; M.nSlow[1] = 0;
-            for (int q = 0; q < 8; ++q) M.stat[q] = 0;
+            for (int q = 0; q < 10; ++q) M.stat[q] = 0;
         }
         __syncthreads();
         if (!prefetched) {
@@ -1132,7 +1183,7 @@ template <bool FAST> __global__ void MV_VIEW_BOUNDS viewKernel(const __grid_cons
                     ++batch;
                     again = true;
                     __syncthreads();
-                    if (tid == 0) { M.nTris = 0; M.nValid = 0x7fffffff; M.tileCtr = 0; }
+                    if (tid == 0) { M.nTris = 0; M.nValid = 0x7fffffff; }
                     __syncthreads();
                 }
             }
@@ -1144,52 +1195,16 @@ template <bool FAST> __global__ void MV_VIEW_BOUNDS viewKernel(const __grid_cons
             atomicAdd(P.consumed + env, 1u);
         }
         const long long tc2 = P.stats ? clock64() : 0;
-        // Claim the next work item now and, if its env's state is already published, fetch its view matrix, its counts and its first
-        // instance chunk while this item's tiles are drawn (the stage buffers, M.view and M.counts are idle during the tile pass): the
-        // global round trips of the item head then cost nothing.  One thread; its warp joins the tile pass a little later.
-        if (tid == 0) {
-            const uint32_t nc = claimWork(P, total);
-            int pre = 0;
-            if (nc < total) {
-                const int nview = P.viewBase + int(nc / uint32_t(bands)), nenv = nview / P.A;
-                bool ready = true;
-                if (P.ready) {
-                    uint32_t v;
-                    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(P.ready + nenv) : "memory");
-                    ready = v == P.readyStamp;
-                    if (ready) asm volatile("fence.proxy.async;" ::: "memory");
-                }
-                if (ready) {
-                    float vm[16];
-                    int32_t cn[8];
-#pragma unroll
-                    for (int q = 0; q < 16; ++q) vm[q] = __ldcg(P.views + size_t(nview) * 16 + q);
-#pragma unroll
-                    for (int q = 0; q < 8; ++q) cn[q] = __ldcg(P.instCounts + nenv * 8 + q);
-#pragma unroll
-                    for (int q = 0; q < 16; ++q) M.view[q] = vm[q];
-#pragma unroll
-                    for (int q = 0; q < 8; ++q) M.counts[q] = cn[q];
-                    if (cn[1] > 0) {
-                        const uint32_t bytes = uint32_t(min(cn[1], kInstChunk)) * uint32_t(sizeof(MvInstance));
-                        mbarExpectTx(&M.bar[0], bytes);
-                        bulkG2S(stage, P.instances + size_t(nenv) * size_t(P.instStride), bytes, &M.bar[0]);
-                    }
-                    pre = 1;
-                }
-            }
-            M.claim = nc; M.prefetched = pre;
-        }
         tilePass<FAST>(P, min(M.nTris, M.nValid), spill, view, rowLo, bandTiles, batch, true);
         __syncthreads();
         if (P.sliceDone && tid == 0) { __threadfence(); atomicAdd(P.sliceDone + env / P.envsPerSlice, 1u); }
         if (P.viewCost && tid == 0) P.viewCost[claim] = uint32_t(min((unsigned long long)clock64() - M.itemStart, 0xffffffffull * 16ull) >> 4);
-        if (P.stats && tid < 8) {
+        if (P.stats && tid < 10) {
             unsigned long long v = M.stat[tid];
             if (tid == 0) v = 1;
             if (tid == 5) v += (unsigned long long)min(M.nTris, M.nValid);
             if (tid == 6) v = (unsigned long long)(batch + 1);
-            atomicAdd(P.stats + tid, v);
+            atomicAdd(P.stats + (tid < 8 ? tid : tid + 6), v);
             if (tid == 0) {
                 const long long tc3 = clock64();
                 atomicAdd(P.stats + 8, (unsigned long long)(tc1 - tc0)); atomicAdd(P.stats + 9, (unsigned long long)tcWait);
